@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- explained-nodes/sec of the GNNExplainer mask-optimisation hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload = BASELINE.json configs[1]: syn1 BA-House (N=700, 2055 edges, d=10, 4 classes; the graph and the trained
@@ -126,7 +126,7 @@ def main_reference(a):
     NN = 871 if a.workload == "syn4" else 700
     workload = WORKLOAD if a.workload != "syn4" else "syn4 Tree-Cycle, explain all 871 nodes batched, 100 epochs, 3-hop subgraphs"
     sample = cpu_sample_nodes(max(2 * procs, 16), NN)
-    steps = max(1, min(a.steps, 2))  # each step is one bounded sample; worker warm-up is inside run_cpu_pool
+    steps = a.steps  # each step is one bounded sample; worker warm-up is inside run_cpu_pool
     vals = []
     for _ in range(steps):
         v, dt = run_cpu_pool(sample, procs)
@@ -392,7 +392,28 @@ def timed(c, fn, steps, warmup, sampler=None, after=None):
     return float(t.item()), extra, wall, clocks
 
 
-def bench_nodes(a, c, name, with_cpu=True, sampler=None):
+DUMP_BYTES = 60 << 20      # --dump-outputs stays below 64 MB in all (npy headers included)
+
+
+def write_outputs(path, arrays, seed=0):
+    """--dump-outputs: arrays[name] -> path/<name>.npy, float32 arrays as float32 and every other array as float64 (exact for the
+    int32 / int64 plan arrays).  When the arrays hold more than DUMP_BYTES, each keeps a share of the budget proportional to its size:
+    the values at sorted, unique positions drawn from a generator seeded with `seed`, so two runs with the same arguments write the
+    same positions; the positions go to path/<name>_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v).ravel() for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    for name, v in arrays.items():
+        if total > DUMP_BYTES:
+            k = int(DUMP_BYTES * v.nbytes / total) // (v.itemsize + 8)      # each kept value also stores its float64 position
+            idx = np.unique(np.random.default_rng(seed).integers(0, v.size, k))
+            np.save(os.path.join(path, name + "_index.npy"), idx.astype(np.float64))
+            v = v[idx]
+        np.save(os.path.join(path, name + ".npy"), v)
+
+
+def bench_nodes(a, c, name, with_cpu=True, sampler=None, dump=None):
     """syn1 / syn4 on ONE GPU through the C ABI: device-resident value + host-buffer e2e."""
     import ctypes as C
     import torch
@@ -434,6 +455,11 @@ def bench_nodes(a, c, name, with_cpu=True, sampler=None):
     l0 = eng.launch_count()
     ms_dev, kern, wall, clocks = timed(c, step_device, a.steps, a.warmup, sampler, after=eng.last_explain_ms)
     launches = (eng.launch_count() - l0) * a.steps // (a.steps + a.warmup)
+    if dump:      # the masks of the last timed step and the subgraph description its plan holds
+        torch.cuda.synchronize(c.dev)
+        p = eng.fetch_plan(nodes)
+        write_outputs(dump, {"masks": out_dev.cpu().numpy(), "node_off": p.node_off, "edge_off": p.edge_off, "neighbors": p.neighbors,
+                             "node_idx_new": p.node_idx_new, "sub_rowptr": p.sub_rowptr, "sub_col": p.sub_col})
     ms_e2e, _, _, _ = timed(c, step_e2e, a.steps, max(3, a.warmup))
     kern_ms = float(np.mean(kern))
     peak, peak_src = _peak_hbm()
@@ -503,7 +529,7 @@ def bench_python_dropin(c, g, reps=3):
     return res
 
 
-def bench_sharded(a, c):
+def bench_sharded(a, c, dump=None):
     """N > 1: gnnx.dist.explain_nodes_sharded (count -> cost-balanced shards -> explain -> ONE all-gather -> unshard)."""
     import torch
     import torch.distributed as dist
@@ -527,6 +553,8 @@ def bench_sharded(a, c):
         if key == "weak":
             res[key]["clocks"] = clocks
             res[key]["wall"] = wall
+            if dump and c.rank == 0:      # every rank holds the gathered masks of the whole list
+                write_outputs(dump, {"masks": keep["out"][0].cpu().numpy(), "edge_off": keep["out"][1]})
     # the strong-scaled 700-node list again in latency mode (gx_debug_set_cluster(h, 0, 0)): a shard leaves SMs idle, so its most expensive
     # tasks run on thread-block clusters; masks agree with the default mode to round-off, not bit for bit, hence opt-in
     ex.engine.debug_cluster(0, 0)
@@ -569,7 +597,7 @@ def main_ours(a):
     c = gpu_ctx(a)
     if a.workload in ("syn1", "syn4") and c.world == 1:
         sampler = ClockSampler(c.local_rank)
-        line, g = bench_nodes(a, c, a.workload, with_cpu=not a.no_cpu, sampler=sampler)
+        line, g = bench_nodes(a, c, a.workload, with_cpu=not a.no_cpu, sampler=sampler, dump=a.dump_outputs)
         if a.workload == "syn1":
             try:
                 line["e2e_python"] = bench_python_dropin(c, g)
@@ -588,7 +616,7 @@ def main_ours(a):
         print(json.dumps(line), flush=True)
         return
     # N > 1
-    g, res, ident, sum_e, sum_n = bench_sharded(a, c)
+    g, res, ident, sum_e, sum_n = bench_sharded(a, c, dump=a.dump_outputs)
     if c.rank == 0:
         w = res["weak"]
         peak, peak_src = _peak_hbm()
@@ -618,7 +646,7 @@ def main_ours(a):
     dist.destroy_process_group()
 
 
-def bench_graphs(a, c, with_cpu=True):
+def bench_graphs(a, c, with_cpu=True, dump=None):
     """BASELINE configs[3] stand-in (Mutagenicity is not in the image): 4337 padded molecule-like graphs, graph-level masks."""
     import ctypes as C
     import torch
@@ -648,6 +676,8 @@ def bench_graphs(a, c, with_cpu=True):
 
     l0 = eng.launch_count()
     ms_dev, kern, _, _ = timed(c, step_dev, a.steps, a.warmup, after=eng.last_explain_ms)
+    if dump:
+        write_outputs(dump, {"masks": out_dev.cpu().numpy(), "edge_off": edge_off})
     launches = (eng.launch_count() - l0) * a.steps // (a.steps + a.warmup)      # this library's kernels inside the timed region (counted by the handle)
     ms_e2e, _, _, _ = timed(c, step_e2e, a.steps, a.warmup)
     kern_ms = float(np.mean(kern))
@@ -668,7 +698,7 @@ def bench_graphs(a, c, with_cpu=True):
     return line
 
 
-def bench_c5(a, c):
+def bench_c5(a, c, dump=None):
     """BASELINE configs[4]: BA(N, m) d=128, 3-hop neighbourhood ~ the whole graph, every task in the streaming kernel; a step explains
     --c5-nodes nodes (default one per SM).  Includes a parity check AT THIS SCALE: a few epochs of one or two of the explained nodes
     against the fp64 sparse edge-list specification (oracle/kernel_spec.py, pinned to the reference through the chain in tests/test_oracle.py)."""
@@ -743,6 +773,8 @@ def bench_c5(a, c):
     sampler.end()
     clocks = sampler.stop()
     c5_launches = eng.launch_count() - l0
+    if dump:
+        write_outputs(dump, {"masks": out_host.numpy()})
     # top-k delivery instead of the full masks (the multi-GPU gather policy for this configuration: denoise_graph(threshold_num=20))
     td0 = time.perf_counter()
     thr, cnt, slots, vals = eng.denoise_topk(out_host.numpy(), 20)
@@ -788,10 +820,13 @@ def main_reference_graphs(a):
     jobs = [(adj[g], feat[g], label[g], W, 100 + g) for g in sample]
     with mp.get_context("fork").Pool(procs) as pool:
         pool.map(_cpu_graph_one, jobs[:procs], chunksize=1)
-        t0 = time.perf_counter(); pool.map(_cpu_graph_one, jobs, chunksize=1); dt = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        for _ in range(a.steps):
+            pool.map(_cpu_graph_one, jobs, chunksize=1)
+        dt = (time.perf_counter() - t0) / a.steps
     v = len(sample) / dt
     print(json.dumps({"impl": "reference", "metric": "explained-graphs/sec (100 mask-opt epochs each)", "value": v, "unit": "graphs/s",
-                      "n_gpus": 1, "steps": 1, "warmup": 0, "ms_per_step": 1000 * dt, "higher_is_better": True, "scaling": "weak",
+                      "n_gpus": 1, "steps": a.steps, "warmup": 0, "ms_per_step": 1000 * dt, "higher_is_better": True, "scaling": "weak",
                       "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                       "config": {"workload": "configs[3] stand-in: %d padded graphs (max_nodes 100, d=14), graph-level mask" % G,
                                  "sample": "%d graphs, %d single-thread worker processes" % (len(sample), procs)},
@@ -813,7 +848,11 @@ if __name__ == "__main__":
     ap.add_argument("--c5-nodes", type=int, default=148, help="explained nodes per step of the c5 workload")
     ap.add_argument("--c5-parity", type=int, default=1, help="nodes checked against the fp64 sparse specification at full scale (0 = skip)")
     ap.add_argument("--cpu-procs", type=int, default=0, help="worker processes of the CPU baseline (default min(cores,64))")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl ours: after the timed steps, write what the last one computed (masks, subgraph description) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if a.impl == "reference":
         if a.workload == "graphs":
             main_reference_graphs(a)
@@ -821,9 +860,9 @@ if __name__ == "__main__":
             main_reference(a)
     elif a.workload == "graphs":
         c = gpu_ctx(a)
-        print(json.dumps(bench_graphs(a, c, with_cpu=not a.no_cpu)), flush=True)
+        print(json.dumps(bench_graphs(a, c, with_cpu=not a.no_cpu, dump=a.dump_outputs)), flush=True)
     elif a.workload == "c5":
         c = gpu_ctx(a)
-        print(json.dumps(bench_c5(a, c)), flush=True)
+        print(json.dumps(bench_c5(a, c, dump=a.dump_outputs)), flush=True)
     else:
         main_ours(a)

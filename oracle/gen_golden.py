@@ -1,7 +1,7 @@
 """gen_golden.py -- generates tests/golden/*.npz by EXECUTING THE UNMODIFIED REFERENCE.
 
 Run in the authoring container only (needs /root/reference):
-    python oracle/gen_golden.py [--only syn1|syn4|rand|graph]
+    python oracle/gen_golden.py [--only syn1|syn4|rand|graph|auc|grad|denoise|teacher|trace|opts|variants|options|tu]
 
 What is pinned (SURVEY.md section 8c: the reference has no tests of its own, so the
 only possible pin is the reference's own output under a fixed seed):
@@ -392,6 +392,64 @@ def gen_variants(R, epochs=30):
     print("  variants golden written")
 
 
+def gen_options(R, node=5, seed=77, epochs=12):
+    """--mask-bias and --mask-act ReLU (SURVEY 8 f3; explain.py:657-660,673-676,755-770): the unmodified reference on a BA(40, 2)
+    graph with a randomly initialised model, run with the default options, with --mask-bias and with --mask-act ReLU under the same
+    seed -> tests/golden/options_golden.npz (graph, weights, M0 at the edges and the three returned (n, n) masks)."""
+    import networkx as nx
+    rng = np.random.default_rng(3)
+    G = nx.barabasi_albert_graph(40, 2, seed=5)
+    N, d, C = 40, 8, 3
+    adj = nx.to_numpy_array(G)[None]
+    feat = rng.normal(size=(1, N, d))
+    label = rng.integers(0, C, size=(1, N))
+    torch.manual_seed(2)
+    model = R.models.GcnEncoderNode(d, 20, 20, C, 3, bn=False, args=train_args(input_dim=d))
+    model.eval()
+    with torch.no_grad():
+        pred, _ = model(torch.tensor(feat, dtype=torch.float), torch.tensor(adj, dtype=torch.float))
+    cg = dict(adj=adj, feat=feat, label=label, pred=pred.numpy(), train_idx=list(range(N)))
+    gold = explain_nodes_ref(R, model, cg, ref_harness.explainer_args(dataset="opt", num_epochs=epochs), [node], seed_base=seed - node)
+    out = dict(N=np.int64(N), edges=edges_of(adj[0]), feat=feat[0], label=label[0].astype(np.int64), pred=cg["pred"][0].astype(np.float32),
+               node=np.int64(node), num_epochs=np.int64(epochs), **state_to_np(model), **gold)
+    for tag, over in (("default", {}), ("mask_bias", dict(mask_bias=True)), ("relu", dict(mask_act="ReLU"))):
+        args = ref_harness.explainer_args(dataset="opt", num_epochs=epochs, **over)
+        with ref_harness.quiet():
+            ex = R.explain.Explainer(model=model, adj=cg["adj"], feat=cg["feat"], label=cg["label"], pred=cg["pred"],
+                                     train_idx=cg["train_idx"], args=args, writer=None, print_training=False, graph_idx=-1)
+            torch.manual_seed(seed)
+            out[tag + "_mask"] = np.asarray(ex.explain(node, graph_idx=0), np.float32)
+    np.savez_compressed(os.path.join(OUT, "options_golden.npz"), **out)
+    print("  option-variant golden written")
+
+
+def gen_tu(R, max_nodes=10):
+    """utils/io_utils.read_graphfile (io_utils.py:426-562) of the unmodified reference on the toy TU-format dataset that
+    tests/util.write_tu_toy writes with seed 4 -> tests/golden/tu_golden.npz: per graph kept, the adjacency padded to max_nodes
+    (diagonal zeroed), the graph label and the node features."""
+    import tempfile
+    import networkx as nx
+    sys.path.insert(0, os.path.join(os.path.dirname(HERE), "tests"))
+    import util
+    with tempfile.TemporaryDirectory() as tmp:
+        util.write_tu_toy(tmp, "TOY", np.random.default_rng(4))
+        ver, nx.__version__ = nx.__version__, "2.5"      # the reference parses the version as a float (io_utils.py:551)
+        try:
+            graphs = R.io_utils.read_graphfile(tmp, "TOY", max_nodes=max_nodes)
+        finally:
+            nx.__version__ = ver
+    out = dict(count=np.int64(len(graphs)))
+    for g, Gx in enumerate(graphs):
+        n = Gx.number_of_nodes()
+        A = np.zeros((max_nodes, max_nodes)); A[:n, :n] = nx.to_numpy_array(Gx)
+        np.fill_diagonal(A, 0)
+        out["g%d_adj" % g] = A
+        out["g%d_label" % g] = np.int64(Gx.graph["label"])
+        out["g%d_feat" % g] = np.array([np.asarray(Gx.nodes[u]["label"], np.float32) for u in Gx.nodes()])
+    np.savez_compressed(os.path.join(OUT, "tu_golden.npz"), **out)
+    print("  TU-reader golden written: %d graphs" % len(graphs))
+
+
 OPT_VARIANTS = (("sgd", dict(opt="sgd")), ("rmsprop", dict(opt="rmsprop")), ("adagrad", dict(opt="adagrad")),
                 ("adamstep", dict(opt="adam", opt_scheduler="step", opt_decay_step=8, opt_decay_rate=0.5)),
                 ("adamcos", dict(opt="adam", opt_scheduler="cos", opt_restart=12)),
@@ -586,6 +644,12 @@ def main():
     if a.only == "graph":
         torch.set_num_threads(8)
         gen_graph_mode(ref_harness.load())
+        return
+    if a.only == "options":
+        gen_options(ref_harness.load())
+        return
+    if a.only == "tu":
+        gen_tu(ref_harness.load())
         return
     if a.short:
         torch.set_num_threads(8)

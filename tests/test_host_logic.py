@@ -97,57 +97,23 @@ def test_make_pred_real_matches_reference():
         assert abs(roc_auc_score(np.concatenate(reals), np.concatenate(preds)) - float(au[which + "_auc"])) < 1e-12
 
 
-def _write_tu(tmp, name, rng):
-    import os
-    os.makedirs(os.path.join(tmp, name), exist_ok=True)
-    pre = os.path.join(tmp, name, name)
-    sizes = [5, 9, 3, 12, 7]
-    gi, nl, A = [], [], []
-    base = 1
-    for g, n in enumerate(sizes, 1):
-        gi += [g] * n
-        nl += list(rng.integers(3, 8, n))
-        perm = rng.permutation(n)
-        es = [(base + int(perm[i]), base + int(perm[i + 1])) for i in range(n - 1)] + [(base + int(rng.integers(0, n)), base + int(rng.integers(0, n))) for _ in range(2)]
-        for a, b in es:
-            if a != b:
-                A += [(a, b), (b, a)]
-        base += n
-    open(pre + "_graph_indicator.txt", "w").write("\n".join(map(str, gi)) + "\n")
-    open(pre + "_node_labels.txt", "w").write("\n".join(map(str, nl)) + "\n")
-    open(pre + "_graph_labels.txt", "w").write("\n".join(map(str, [1, -1, -1, 1, 1])) + "\n")
-    open(pre + "_A.txt", "w").write("\n".join("%d, %d" % e for e in A) + "\n")
-    return sizes
-
-
 def test_tu_reader_matches_reference(tmp_path):
-    """gnnx.io_utils.read_tu_dataset against the reference's read_graphfile + padding (authoring container only;
-    on a box without /root/reference the structural checks still run)."""
+    """gnnx.io_utils.read_tu_dataset against what the reference's read_graphfile + padding returned on the same toy dataset
+    (tests/golden/tu_golden.npz, oracle/gen_golden.py --only tu)."""
     from gnnx.io_utils import read_tu_dataset
     rng = np.random.default_rng(4)
-    sizes = _write_tu(str(tmp_path), "TOY", rng)
+    sizes = util.write_tu_toy(str(tmp_path), "TOY", rng)
     out = read_tu_dataset(str(tmp_path), "TOY", max_nodes=10)
     assert out["adj"].shape[1:] == (10, 10) and len(out["label"]) == 4            # the 12-node graph is dropped
     assert np.array_equal(out["adj"], out["adj"].transpose(0, 2, 1)) and out["feat"].shape[2] == 5
     assert list(out["label"]) == [0, 1, 1, 0]                                      # first-appearance renumbering of {1,-1}
-    import ref_harness
-    if not ref_harness.available():
-        return
-    R = ref_harness.load()
-    import networkx as nx
-    ver, nx.__version__ = nx.__version__, "2.5"      # the reference parses the version as a float (io_utils.py:551)
-    try:
-        graphs = R.io_utils.read_graphfile(str(tmp_path), "TOY", max_nodes=10)
-    finally:
-        nx.__version__ = ver
-    assert len(graphs) == len(out["label"])
-    for g, Gx in enumerate(graphs):
-        n = Gx.number_of_nodes()
-        A = np.zeros((10, 10)); A[:n, :n] = nx.to_numpy_array(Gx)
-        np.fill_diagonal(A, 0)
-        assert np.array_equal(A, out["adj"][g]) and int(Gx.graph["label"]) == int(out["label"][g])
-        for i, u in enumerate(Gx.nodes()):
-            assert np.array_equal(np.asarray(Gx.nodes[u]["label"], dtype=np.float32), out["feat"][g, i])
+    ref = np.load(os.path.join(util.GOLDEN, "tu_golden.npz"))
+    assert int(ref["count"]) == len(out["label"])
+    for g in range(len(out["label"])):
+        assert np.array_equal(ref["g%d_adj" % g], out["adj"][g]) and int(ref["g%d_label" % g]) == int(out["label"][g])
+        feat = ref["g%d_feat" % g]
+        assert len(feat) == [s for s in sizes if s <= 10][g]
+        assert np.array_equal(feat, out["feat"][g, :len(feat)])
 
 
 def test_bench_ba_generator_is_a_simple_symmetric_graph():

@@ -140,47 +140,33 @@ def test_graph_mode_oracle_matches_reference():
 
 
 def test_reference_option_variants_mask_bias_noop_and_relu_nan():
-    """SURVEY 8(f3) option variants, pinned by executing the reference (authoring container only):
+    """SURVEY 8(f3) option variants, pinned by the masks the unmodified reference returned with the default options, with
+    --mask-bias and with --mask-act ReLU under one seed (tests/golden/options_golden.npz, oracle/gen_golden.py --only options):
       * --mask-bias: the bias matrix starts at 0, passes through ReLU6(6 b)/6 whose gradient at exactly 0 is 0, so Adam
         never moves it and the returned mask is BIT-IDENTICAL to the default run (explain.py:657-660,673-676) -- which is
         why the engine accepts the flag as a no-op;
       * --mask-act ReLU: the entropy regulariser takes log(1 - relu(M)) with M ~ N(1, 2/n) (explain.py:755-770), i.e. the
         log of a negative number for about half the entries: the loss and every returned mask entry are NaN from the first
-        step -- nothing to build against."""
-    import ref_harness
-    if not ref_harness.available():
-        pytest.skip("reference tree not present")
-    import torch
-    import networkx as nx
-    R = ref_harness.load()
-    rng = np.random.default_rng(3)
-    G = nx.barabasi_albert_graph(40, 2, seed=5)
-    N, d, C = 40, 8, 3
-    adj = nx.to_numpy_array(G)[None]
-    feat = rng.normal(size=(1, N, d))
-    label = rng.integers(0, C, size=(1, N))
-    torch.manual_seed(2)
-    import gen_golden
-    model = R.models.GcnEncoderNode(d, 20, 20, C, 3, bn=False, args=gen_golden.train_args(input_dim=d))
-    model.eval()
-    with torch.no_grad():
-        pred, _ = model(torch.tensor(feat, dtype=torch.float), torch.tensor(adj, dtype=torch.float))
-    cg = dict(adj=adj, feat=feat, label=label, pred=pred.numpy(), train_idx=list(range(N)))
-
-    def run(**over):
-        args = ref_harness.explainer_args(dataset="opt", num_epochs=12, **over)
-        with ref_harness.quiet():
-            ex = R.explain.Explainer(model=model, adj=cg["adj"], feat=cg["feat"], label=cg["label"], pred=cg["pred"],
-                                     train_idx=cg["train_idx"], args=args, writer=None, print_training=False, graph_idx=-1)
-            torch.manual_seed(77)
-            return np.asarray(ex.explain(5, graph_idx=0))
-
-    base = run()
+        step -- nothing to build against.
+    The torch port, run on the same graph, weights and M0, reproduces the default run."""
+    g = np.load(util.GOLDEN + "/options_golden.npz")
+    node = int(g["node"])
+    base = g["default_mask"]
     assert np.isfinite(base).all() and base.max() > 0
-    assert np.array_equal(run(mask_bias=True), base)
-    relu = run(mask_act="ReLU")
+    assert np.array_equal(g["mask_bias_mask"], base)
+    relu = g["relu_mask"]
     ei, ej = np.nonzero(base)
     assert np.isnan(relu[ei, ej]).all()
+    rowptr, col = O.csr_from_edges(int(g["N"]), g["edges"])
+    idx, srp, scol, sfeat, slabel, nbrs = O.extract_neighborhood(rowptr, col, g["feat"], g["label"], node, 3)
+    assert np.array_equal(nbrs, g["n%d_nbrs" % node]) and idx == int(g["n%d_idx_new" % node])
+    A = O.dense_from_csr(srp, scol)
+    ei, ej = np.nonzero(A)
+    M0 = np.ones_like(A, dtype=np.float32); M0[ei, ej] = g["n%d_m0" % node]
+    port = O.explain_dense_torch(A, sfeat, slabel[idx], np.argmax(g["pred"], 1)[nbrs], idx, {k: g[k] for k in util.WKEYS}, M0,
+                                 hp=O.default_hparams(num_epochs=int(g["num_epochs"])))
+    assert np.array_equal(base[ei, ej], g["n%d_mask" % node])
+    assert O.rel_l2(port[ei, ej], base[ei, ej]) < 1e-6
 
 
 def test_grad_baseline_oracle_matches_reference_golden():

@@ -65,6 +65,29 @@ def assert_per_node(errs, name, epochs):
     return tol
 
 
+def write_tu_toy(tmp, name, rng):
+    """Five small graphs in the TU graph-kernel text format under tmp/name/ (one of 12 nodes); returns their sizes."""
+    os.makedirs(os.path.join(tmp, name), exist_ok=True)
+    pre = os.path.join(tmp, name, name)
+    sizes = [5, 9, 3, 12, 7]
+    gi, nl, A = [], [], []
+    base = 1
+    for g, n in enumerate(sizes, 1):
+        gi += [g] * n
+        nl += list(rng.integers(3, 8, n))
+        perm = rng.permutation(n)
+        es = [(base + int(perm[i]), base + int(perm[i + 1])) for i in range(n - 1)] + [(base + int(rng.integers(0, n)), base + int(rng.integers(0, n))) for _ in range(2)]
+        for a, b in es:
+            if a != b:
+                A += [(a, b), (b, a)]
+        base += n
+    open(pre + "_graph_indicator.txt", "w").write("\n".join(map(str, gi)) + "\n")
+    open(pre + "_node_labels.txt", "w").write("\n".join(map(str, nl)) + "\n")
+    open(pre + "_graph_labels.txt", "w").write("\n".join(map(str, [1, -1, -1, 1, 1])) + "\n")
+    open(pre + "_A.txt", "w").write("\n".join("%d, %d" % e for e in A) + "\n")
+    return sizes
+
+
 def rel_l2(a, b):
     a = np.asarray(a, np.float64).ravel()
     b = np.asarray(b, np.float64).ravel()
