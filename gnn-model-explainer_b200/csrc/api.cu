@@ -60,11 +60,12 @@ constexpr int kNumClasses = sizeof(kClasses) / sizeof(kClasses[0]);
 constexpr int kStreamClass = 5;    // explain_stream.cu: state in a global slab
 constexpr int kClusterClass = 6;   // explain_node.cu with a thread-block cluster per task: the most expensive shared-memory tasks
 constexpr int kOneClass = 4, kTwoClass = 3;
+constexpr int64_t kGraphVarSmallWords = 64 * 1024;   // explain_graph_var.cu: slabs up to 256 KB form the small-slab class
 // Cluster class (gx_debug_set_cluster / GNNX_CLUSTER_SIZE): off by default, so that a task's masks never depend on the batch it is in;
 // 0 = latency mode, gx_plan_nodes moves the most expensive tasks of a batch that leaves SMs idle to clusters; 2 / 4 = every task above
 // cluster_cost.  A full 700-node batch is throughput bound: splitting its tasks only adds barrier and DSMEM overhead
 // (profiles/r02a_bench_cluster_default_on_REJECTED.json), so the latency mode gives it none.
-constexpr int kNumStreams = kNumClasses;
+constexpr int kNumStreams = kNumClasses + 1;   // graph mode: 6 shared-memory classes + 2 classes of explain_graph_var.cu
 
 }  // namespace
 
@@ -128,6 +129,11 @@ struct gx_handle {
   int g_max_smem = 0, g_max_np = 0;
   // graph mode launch classes (by shared-memory footprint, like node mode): tasks per class, the class's largest footprint / pair count
   int g_class_n[6] = {}, g_class_smem[6] = {}, g_class_np[6] = {};
+  // explain_graph_var.cu classes (small / large slab) per routing: [0] the batch with Adam (tasks the shared-memory kernel does not
+  // take), [1] the whole batch (optimisers other than Adam); their task ids follow the shared-memory classes in d_order ([0]) or
+  // fill d_order[count, 2 count) ([1]); words = the class's largest slab
+  int gv_n[2][2] = {}, gv_off[2] = {};
+  int64_t gv_words[2][2] = {};
   // slot workspace
   DevBuf ws_buf;
   GxSlotWs ws{};
@@ -1169,13 +1175,18 @@ int gx_set_graph_batch_csr(gx_handle* h, int32_t G, int32_t max_nodes, const int
 int gx_plan_graphs(gx_handle* h, const int32_t* graph_ids, int32_t count, int64_t* edge_off, int64_t* total_edges) {
   if (!h || !graph_ids) { gx_set_error("gx_plan_graphs: NULL argument"); return GX_ERR_INVALID; }
   if (!h->has_batch || !h->has_model) { gx_set_error("gx_plan_graphs: call gx_set_model and gx_set_graph_batch_csr first"); return GX_ERR_INVALID; }
-  if (h->m.variant) { gx_set_error("gx_plan_graphs: graph mode builds the default model only (3 layers, no --bn)"); return GX_ERR_UNSUPPORTED; }
   if (h->gb.d != h->m.d) { gx_set_error("gx_plan_graphs: feat_dim %d != model input_dim %d", h->gb.d, h->m.d); return GX_ERR_INVALID; }
   if (count <= 0) { gx_set_error("gx_plan_graphs: count <= 0"); return GX_ERR_INVALID; }
+  if (gx_graph_var_smem_bytes(h->m.d, h->m.L, h->m.hid, h->m.emb, h->m.C) > gx_explain_max_smem()) {
+    gx_set_error("gx_plan_graphs: model does not fit the shared memory of the graph-mode variant kernel"); return GX_ERR_UNSUPPORTED;
+  }
   GX_CUDA_CHECK(cudaSetDevice(h->device));
   h->has_gplan = false; h->has_plan = false;
   const int nf = h->gb.max_nodes;
+  const int vw = gx_graph_var_row_stride(h->m.hid, h->m.emb);
   h->tasks.assign(count, GxTask());
+  std::vector<int64_t> var_words(count);
+  std::vector<char> in_smem(count);
   int64_t tn = 0, te = 0, tp = 0;
   int max_smem = 0, max_np = 0;
   const int nwarps = 128 / 32;
@@ -1191,11 +1202,18 @@ int gx_plan_graphs(gx_handle* h, const int32_t* graph_ids, int32_t count, int64_
     T.e_d = rp[nf] - rp[0]; T.e1 = T.e_d; T.npairs = T.e_d / 2; T.npairs_in = T.npairs;
     T.gt_label = h->gb_h_label[g]; T.n_norm = nf; T.flags = na < nf ? 1 : 0;
     T.node_off = tn; T.rp_off = tn + t; T.edge_off = te; T.pair_off = tp;
-    if (na >= 65535 || T.e_d >= 65535) { gx_set_error("gx_plan_graphs: graph %d too large for the shared-memory kernel", g); return GX_ERR_UNSUPPORTED; }
-    const GxLayoutG L = gx_make_layout_graph(na, T.e_d, T.npairs, h->m.d, h->m.hid, h->m.emb, h->m.C, nwarps);
-    T.smem_bytes = L.total_words * 4;
-    if (T.smem_bytes > 226 * 1024) { gx_set_error("gx_plan_graphs: graph %d needs %d bytes of shared memory", g, T.smem_bytes); return GX_ERR_UNSUPPORTED; }
-    max_smem = std::max(max_smem, T.smem_bytes); max_np = std::max(max_np, T.npairs);
+    var_words[t] = gx_make_graph_var_layout(na, T.e_d, T.npairs, h->m.d, h->m.L, vw).total_words;
+    // the tuned shared-memory kernel takes the default model's graphs that fit its layout (16-bit indices, 226 KB); the rest goes to
+    // explain_graph_var.cu
+    in_smem[t] = !h->m.variant && na < 65535 && T.e_d < 65535;
+    if (in_smem[t]) {
+      const GxLayoutG L = gx_make_layout_graph(na, T.e_d, T.npairs, h->m.d, h->m.hid, h->m.emb, h->m.C, nwarps);
+      T.smem_bytes = L.total_words * 4;
+      in_smem[t] = T.smem_bytes <= 226 * 1024;
+    }
+    if (!in_smem[t]) T.smem_bytes = 0;
+    else max_smem = std::max(max_smem, T.smem_bytes);
+    max_np = std::max(max_np, T.npairs);
     tn += na; te += T.e_d; tp += T.npairs;
   }
   // Launch classes by footprint: a batch padded to 100 nodes mostly holds 20-40-node molecules; one launch sized for the largest graph
@@ -1205,24 +1223,42 @@ int gx_plan_graphs(gx_handle* h, const int32_t* graph_ids, int32_t count, int64_
   std::vector<int32_t> cls_tasks[6];
   for (int c = 0; c < 6; ++c) { h->g_class_n[c] = 0; h->g_class_smem[c] = 0; h->g_class_np[c] = 0; }
   for (int t = 0; t < count; ++t) {
+    if (!in_smem[t]) continue;
     int c = 0;
     while (c < 5 && h->tasks[t].smem_bytes > kGraphCap[c]) ++c;
     cls_tasks[c].push_back(t);
     h->g_class_smem[c] = std::max(h->g_class_smem[c], h->tasks[t].smem_bytes);
     h->g_class_np[c] = std::max(h->g_class_np[c], h->tasks[t].npairs);
   }
+  auto costlier = [&](int32_t x, int32_t y) { return h->tasks[x].e_d + 4 * h->tasks[x].n > h->tasks[y].e_d + 4 * h->tasks[y].n; };
   std::vector<int32_t> order;
-  order.reserve(count);
+  order.reserve(2 * (size_t)count);
   for (int c = 0; c < 6; ++c) {
-    std::stable_sort(cls_tasks[c].begin(), cls_tasks[c].end(), [&](int32_t x, int32_t y) { return h->tasks[x].e_d + 4 * h->tasks[x].n > h->tasks[y].e_d + 4 * h->tasks[y].n; });
+    std::stable_sort(cls_tasks[c].begin(), cls_tasks[c].end(), costlier);
     h->g_class_n[c] = (int)cls_tasks[c].size();
     order.insert(order.end(), cls_tasks[c].begin(), cls_tasks[c].end());
   }
+  // explain_graph_var.cu: a small-slab class (molecules: many CTAs per SM, slabs in L2) and a large-slab class (a few hundred nodes and
+  // more: few CTAs, so that one 4 000-node graph does not size the slab of every CTA of the grid).  Routing [0]: the tasks above;
+  // routing [1]: every task (optimisers other than Adam).
+  for (int r = 0; r < 2; ++r) {
+    std::vector<int32_t> cv[2];
+    for (int t = 0; t < count; ++t)
+      if (r == 1 || !in_smem[t]) cv[var_words[t] > kGraphVarSmallWords ? 1 : 0].push_back(t);
+    h->gv_off[r] = (int)order.size();
+    for (int c = 0; c < 2; ++c) {
+      std::stable_sort(cv[c].begin(), cv[c].end(), costlier);
+      h->gv_n[r][c] = (int)cv[c].size();
+      h->gv_words[r][c] = 4;
+      for (int32_t t : cv[c]) h->gv_words[r][c] = std::max(h->gv_words[r][c], var_words[t]);
+      order.insert(order.end(), cv[c].begin(), cv[c].end());
+    }
+  }
   GX_CUDA_CHECK(h->d_tasks.reserve((size_t)count * sizeof(GxTask)));
   GX_CUDA_CHECK(cudaMemcpyAsync(h->d_tasks.p, h->tasks.data(), (size_t)count * sizeof(GxTask), cudaMemcpyHostToDevice, h->stream));
-  GX_CUDA_CHECK(h->d_order.reserve((size_t)count * 4));
-  GX_CUDA_CHECK(cudaMemcpyAsync(h->d_order.p, order.data(), (size_t)count * 4, cudaMemcpyHostToDevice, h->stream));
-  GX_CUDA_CHECK(h->d_counters.reserve(kNumClasses * 4));
+  GX_CUDA_CHECK(h->d_order.reserve(order.size() * 4));
+  GX_CUDA_CHECK(cudaMemcpyAsync(h->d_order.p, order.data(), order.size() * 4, cudaMemcpyHostToDevice, h->stream));
+  GX_CUDA_CHECK(h->d_counters.reserve(kNumStreams * 4));
   GX_CUDA_CHECK(h->d_lo2gid.reserve((size_t)std::max<int64_t>(tn, 1) * 4));
   GX_CUDA_CHECK(h->d_irp.reserve((size_t)(tn + count) * 4));
   GX_CUDA_CHECK(h->d_icol.reserve((size_t)std::max<int64_t>(te, 1) * 4));
@@ -1252,16 +1288,24 @@ static int explain_graphs_impl(gx_handle* h, const gx_hparams* hp, gx_memspace s
   if (hp->mask_act != 0) { gx_set_error("gx_explain_graphs: mask_act != sigmoid is not built (the reference's ReLU variant returns NaN masks)"); return GX_ERR_UNSUPPORTED; }
   if (hp->num_epochs < 1) { gx_set_error("gx_explain_graphs: num_epochs < 1"); return GX_ERR_INVALID; }
   if (hp->init != GX_INIT_M0 && hp->init != GX_INIT_PHILOX && hp->init != GX_INIT_STATE) { gx_set_error("gx_explain_graphs: unknown init %d", hp->init); return GX_ERR_INVALID; }
+  int rc = check_optimiser("gx_explain_graphs", hp);
+  if (rc != GX_OK) return rc;
+  // routing [1]: optimisers other than Adam run the whole batch in explain_graph_var.cu; [0]: Adam, the variant kernel takes the
+  // tasks explain_graph.cu does not (model variants, graphs beyond its shared-memory layout)
+  const int route = hp->opt != GX_OPT_ADAM ? 1 : 0;
+  const bool any_var = h->gv_n[route][0] + h->gv_n[route][1] > 0;
+  if (any_var && (hp->init == GX_INIT_STATE || (io && (io->trace || io->trace_pred || io->adam_m_out || io->adam_v_out || io->mask_param_out || io->feat_state_out)))) {
+    gx_set_error("gx_explain_graphs: model variants (num_layers != 3 / --bn / widths > 32), optimisers other than Adam and graphs beyond the shared-memory kernel "
+                 "build the mask optimisation only (no trace or optimiser state)");
+    return GX_ERR_UNSUPPORTED;
+  }
   GX_CUDA_CHECK(cudaSetDevice(h->device));
   const int count = h->g_count;
   const int64_t te = h->g_total_e;
   IoDev D;
-  int rc = io_prepare(h, "gx_explain_graphs", hp, 0, space, io, count, te, h->m.d, h->m.C, &D);
+  rc = io_prepare(h, "gx_explain_graphs", hp, 0, space, io, count, te, h->m.d, h->m.C, &D);
   if (rc != GX_OK) return rc;
   D.x.tr_outer = nullptr;   // graph mode has no outer pairs
-  rc = check_optimiser("gx_explain_graphs", hp);
-  if (rc != GX_OK) return rc;
-  if (hp->opt != GX_OPT_ADAM) { gx_set_error("gx_explain_graphs: graph mode builds Adam only (the schedulers work)"); return GX_ERR_UNSUPPORTED; }
   GxHparamsDev hd;
   fill_hparams(h, hp, 0, D.x.trace != nullptr, &hd);
   hd.c_lap = 0.f;           // lap_loss = 0 in graph mode (explain.py:787-788)
@@ -1271,20 +1315,59 @@ static int explain_graphs_impl(gx_handle* h, const gx_hparams* hp, gx_memspace s
   // one persistent launch per footprint class, on its own stream (the classes overlap like the node-mode classes)
   int grids[6]; int64_t pstride[6], poff[7] = {};
   for (int c = 0; c < 6; ++c) {
+    const int nt = route == 0 ? h->g_class_n[c] : 0;
     const int smem_c = std::max(h->g_class_smem[c], 1024);
     const int per_sm = std::max(1, std::min(16, (227 * 1024) / (smem_c + 1024)));
-    grids[c] = std::min(h->g_class_n[c], h->num_sms * per_sm);
+    grids[c] = std::min(nt, h->num_sms * per_sm);
     pstride[c] = ((int64_t)h->g_class_np[c] * 8 + 3) / 4 * 4;
     poff[c + 1] = poff[c] + pstride[c] * grids[c];
   }
   GX_CUDA_CHECK(h->d_pws.reserve((size_t)std::max<int64_t>(poff[6], 4) * 4));
-  GX_CUDA_CHECK(cudaMemsetAsync(h->d_counters.p, 0, kNumClasses * 4, h->stream));
+  // explain_graph_var.cu: one slab per CTA, sized by the class's largest graph; 8 CTAs per SM of 128 threads (fewer when the weights
+  // take the shared memory), the large-slab class 2 per SM and no more than 80% of the free device memory
+  int vgrid[2] = {0, 0}; int64_t voff[3] = {0, 0, 0};
+  if (any_var) {
+    const int vsm = gx_graph_var_smem_bytes(h->m.d, h->m.L, h->m.hid, h->m.emb, h->m.C);
+    const int per_sm = std::max(1, std::min(8, (227 * 1024) / (vsm + 1024)));
+    size_t free_b = 0, total_b = 0;
+    GX_CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
+    const int64_t budget = (int64_t)(free_b + h->d_gws.cap) / 4 * 8 / 10;   // words
+    for (int c = 0; c < 2; ++c) {
+      const int nt = h->gv_n[route][c];
+      voff[c + 1] = voff[c];
+      if (nt == 0) continue;
+      const int64_t words = h->gv_words[route][c];
+      const int64_t room = c == 0 ? budget / 2 : budget - voff[1];   // the small class leaves at least half of the budget to the large one
+      const int grid = (int)std::min<int64_t>(std::min(nt, h->num_sms * (c == 0 ? per_sm : std::min(per_sm, 2))), room / words);
+      if (grid < 1) { gx_set_error("gx_explain_graphs: a graph needs %lld MB of device workspace", (long long)(words * 4 >> 20)); return GX_ERR_CUDA; }
+      vgrid[c] = grid;
+      voff[c + 1] = voff[c] + words * grid;
+    }
+    GX_CUDA_CHECK(h->d_gws.reserve((size_t)std::max<int64_t>(voff[2], 4) * 4));
+  }
+  GX_CUDA_CHECK(cudaMemsetAsync(h->d_counters.p, 0, kNumStreams * 4, h->stream));
   GX_CUDA_CHECK(cudaEventRecord(h->ev_t0, h->stream));
   GX_CUDA_CHECK(cudaEventRecord(h->ev_fork, h->stream));
   int offs[6];
   for (int c = 0, acc = 0; c < 6; ++c) { offs[c] = acc; acc += h->g_class_n[c]; }
+  for (int c = 1; c >= 0; --c) {   // large graphs first
+    if (vgrid[c] == 0) continue;
+    const int sidx = 6 + c;
+    GxExplainLaunch cfg;
+    cfg.order = h->d_order.as<int32_t>() + h->gv_off[route] + (c == 1 ? h->gv_n[route][0] : 0);
+    cfg.ntasks = h->gv_n[route][c]; cfg.counter = h->d_counters.as<int32_t>() + sidx;
+    cfg.smem_bytes = 0; cfg.threads = 0; cfg.grid = vgrid[c];
+    cfg.gws = h->d_gws.as<float>() + voff[c]; cfg.gws_stride_words = h->gv_words[route][c];
+    cfg.pws = nullptr; cfg.pws_stride_words = 0; cfg.dbg = nullptr;
+    cfg.x = D.x;
+    GX_CUDA_CHECK(cudaStreamWaitEvent(h->side[sidx], h->ev_fork, 0));
+    GX_CUDA_CHECK(gx_launch_explain_graph_var(cfg, h->gb, h->m, hd, h->plan, D.m0, D.out, D.feat, h->side[sidx]));
+    GX_CUDA_CHECK(cudaEventRecord(h->ev_join[sidx], h->side[sidx]));
+    GX_CUDA_CHECK(cudaStreamWaitEvent(h->stream, h->ev_join[sidx], 0));
+    h->launches += 1;
+  }
   for (int c = 5; c >= 0; --c) {   // largest graphs first
-    if (h->g_class_n[c] == 0) continue;
+    if (grids[c] == 0) continue;
     GxExplainLaunch cfg;
     cfg.order = h->d_order.as<int32_t>() + offs[c]; cfg.ntasks = h->g_class_n[c]; cfg.counter = h->d_counters.as<int32_t>() + c;
     cfg.smem_bytes = std::max(h->g_class_smem[c], 1024);

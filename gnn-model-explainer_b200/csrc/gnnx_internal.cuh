@@ -223,6 +223,30 @@ __host__ __device__ inline GxVarLayout gx_make_var_layout(int n, int n2, int e1,
   return Lo;
 }
 
+// Global-memory slab of one graph-mode task in explain_graph_var.cu (model variants, optimisers other than Adam, graphs beyond
+// shared memory): every one of the `na` rows with an edge at every layer; hidden-width arrays have row stride vw = 32 * ceil(width / 32).
+struct GxGraphVarLayout {
+  int64_t a, U, dZ1, Yh, H, dZ, q, istd, P;
+  int64_t total_words;
+};
+__host__ __device__ inline GxGraphVarLayout gx_make_graph_var_layout(int na, int e_d, int np, int d, int L, int vw) {
+  GxGraphVarLayout Lo;
+  const int dp = gx_round_up(d, 4);
+  int64_t o = 0;
+  auto take = [&](int64_t words) { int64_t r = o; o += (words + 3) / 4 * 4; return r; };
+  Lo.a = take(e_d);                             // masked adjacency of every internal slot
+  Lo.U = take((int64_t)na * dp);                // A_m X
+  Lo.dZ1 = take((int64_t)na * dp);              // dL/d(A_m X') (.) sigmoid(feat_mask)
+  Lo.Yh = take((int64_t)L * na * vw);           // per layer: normalised pre-activations
+  Lo.H = take((int64_t)L * na * vw);            // per layer: relu (+ standardisation) output = input of the next layer / the max-pool
+  Lo.dZ = take((int64_t)(L - 1) * na * vw);     // layers 2..L: dL/d(A_m H_{l-1})
+  Lo.q = take((int64_t)L * na);
+  Lo.istd = take((int64_t)L * na);
+  Lo.P = take((int64_t)np * 8);                 // per undirected edge: (M, m, v, S) of both directions
+  Lo.total_words = o;
+  return Lo;
+}
+
 // Shared-memory footprint of one graph-mode task (all `na` rows with at least one edge are computed at every layer).
 struct GxLayoutG {
   int X, U, Yh1, Yh2, Yh3, q, dZ2, dZ3, a, W1s, W1t, W2s, W2t, W3s, W3t, bs, cst, emb, dE, sF, F, mF, vF, gFp, zs, logit, Wp;
@@ -340,6 +364,12 @@ cudaError_t gx_launch_graph_plan(const GxGraphBatchDev& gb, int count, GxPlanArr
 cudaError_t gx_launch_explain_graphs(const GxExplainLaunch& cfg, const GxGraphBatchDev& gb, const GxModelDev& m,
                                      const GxHparamsDev& hp, const GxPlanArrays& plan, const float* m0, float* out_mask,
                                      float* out_feat, cudaStream_t s);
+// explain_graph_var.cu: cfg.gws / gws_stride_words = the per-CTA slabs (gx_make_graph_var_layout of the launch's largest task)
+cudaError_t gx_launch_explain_graph_var(const GxExplainLaunch& cfg, const GxGraphBatchDev& gb, const GxModelDev& m,
+                                        const GxHparamsDev& hp, const GxPlanArrays& plan, const float* m0, float* out_mask,
+                                        float* out_feat, cudaStream_t s);
+int gx_graph_var_smem_bytes(int d, int L, int hid, int emb, int C);
+int gx_graph_var_row_stride(int hid, int emb);
 cudaError_t gx_launch_outer_pairs(const GxHparamsDev& hp, const GxGraphDev& g, const GxPlanArrays& plan, int count,
                                   const float* m0, float* out_mask, const GxExtra& x, cudaStream_t s);
 cudaError_t gx_launch_denoise_topk(const GxPlanArrays& plan, int count, const float* edge_mask, int k2, int cap, float* out_thr,

@@ -96,11 +96,9 @@ class Explainer:
         # utils/train_utils.py:7-23: adam / sgd / rmsprop / adagrad, schedulers none / step / cos
         if getattr(args, "opt", "adam") not in _abi.GX_OPT or getattr(args, "opt_scheduler", "none") not in _abi.GX_SCHED:
             raise ValueError("unknown optimiser / scheduler: %r / %r" % (getattr(args, "opt", None), getattr(args, "opt_scheduler", None)))
-        if graph_mode and getattr(args, "opt", "adam") != "adam":
-            raise NotImplementedError("graph mode builds Adam only (the schedulers work)")
+        # graph mode takes every model variant (layers, --bn, widths) and optimiser too: the graphs that explain_graph.cu does not
+        # build run in explain_graph_var.cu
         bn = bool(getattr(model, "bn", False))
-        if bn and graph_mode:
-            raise NotImplementedError("--bn is built for node tasks only")
         if device is None:
             device = int(os.environ.get("LOCAL_RANK", "0")) if torch.cuda.is_available() else 0
         self.engine = Engine(device)

@@ -206,11 +206,16 @@ int gx_grad_nodes(gx_handle* h, gx_memspace space, float* edge_mask);
 int gx_set_graph_batch_csr(gx_handle* h, int32_t num_graphs, int32_t max_nodes, const int32_t* rowptr,
                            const int32_t* col, const float* feat, int32_t feat_dim, const int32_t* label);
 /* Plans the graphs to explain; edge_off[count+1] (may be NULL) receives the packed slot offsets: the slots of
- * graph t are the entries of its adjacency in row-major order (its slice of the CSR). */
+ * graph t are the entries of its adjacency in row-major order (its slice of the CSR).  Every model gx_set_model accepts is
+ * accepted (num_layers 2..4, GX_MODEL_BN, widths up to 128, input_dim <= 128), and every graph up to max_nodes = 4096: the default
+ * model (3 layers, no bn, widths <= 32) on a graph whose state fits 226 KB of shared memory runs in the tuned graph kernel, every
+ * other graph in the graph-mode variant kernel (state in a per-CTA global slab). */
 int gx_plan_graphs(gx_handle* h, const int32_t* graph_ids, int32_t count, int64_t* edge_off, int64_t* total_edges);
 /* Explainer.explain(node_idx=0, graph_idx=g, graph_mode=True) for every planned graph (model =
  * GcnEncoderGraph: per-layer max-pool readout, models.py:269-316; lap_loss = 0, explain.py:787-788).
- * m0_edges / edge_mask: [total_edges] in `space`, as for gx_explain_nodes. */
+ * m0_edges / edge_mask: [total_edges] in `space`, as for gx_explain_nodes.  All four optimisers and both schedulers; with an
+ * optimiser other than Adam the whole batch runs in the variant kernel.  A call in which any graph runs in the variant kernel builds
+ * the mask optimisation only: a trace, GX_INIT_STATE or optimiser-state outputs return GX_ERR_UNSUPPORTED. */
 int gx_explain_graphs(gx_handle* h, const gx_hparams* hp, gx_memspace space, const float* m0_edges,
                       float* edge_mask, float* feat_mask);
 int gx_explain_graphs_ex(gx_handle* h, const gx_hparams* hp, gx_memspace space, const gx_explain_io* io);

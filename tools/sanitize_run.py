@@ -2,7 +2,7 @@
 """Small invocation of every kernel for compute-sanitizer (racecheck / memcheck / synccheck are ~100x slower than a plain run):
     compute-sanitizer --tool racecheck python tools/sanitize_run.py
 k-hop extraction + shared-memory kernel on a mix of task sizes (syn1: hub node 0 and tiny tasks), the streaming kernel (forced),
-the gradient baseline, graph mode, densify, neighbourhood rows.  A few epochs each."""
+the gradient baseline, graph mode (tuned kernel and graph-variant kernel), densify, neighbourhood rows.  A few epochs each."""
 import os
 import sys
 
@@ -19,7 +19,7 @@ EPOCHS = int(os.environ.get("SAN_EPOCHS", "4"))
 
 
 def main():
-    which = sys.argv[1:] or ["node", "stream", "graph", "misc", "var", "cluster"]
+    which = sys.argv[1:] or ["node", "stream", "graph", "graphvar", "misc", "var", "cluster"]
     fx = util.load_fixture("syn1")
     if "node" in which:
         eng = util.make_engine(fx)
@@ -95,6 +95,47 @@ def main():
         out = np.zeros(int(eoff[-1]), np.float32)
         eng.explain_graphs_host(eng.make_hparams(num_epochs=EPOCHS), m0, out)
         print("graph ok", float(out.sum()))
+        eng.close()
+    if "graphvar" in which:
+        # explain_graph_var.cu: 4 layers + bn (small-slab class), a 128-wide model, the default model with sgd, and the default model
+        # on a batch padded to 600 nodes whose largest graph exceeds the shared-memory kernel (large-slab class next to the tuned kernel)
+        g = np.load(util.GOLDEN + "/graphs_golden.npz")
+        gv = np.load(util.GOLDEN + "/graph_variants_golden.npz")
+        gids = [0, 3, 5, 11]
+        m0 = np.concatenate([g["g%d_m0" % i] for i in gids]).astype(np.float32)
+        for tag, L, bn in (("L4bn", 4, True), ("w128", 2, False)):
+            w = {k[len(tag) + 1:]: gv[k] for k in gv.files if k.startswith(tag + "_W") or (k.startswith(tag + "_b") and k != tag + "_bn")}
+            eng = gnnx.Engine(0)
+            eng.set_model(w, num_layers=L, bn=bn)
+            eng.set_graph_batch(g["adj"], g["feat"], g["label"])
+            eoff = eng.plan_graphs(gids)
+            out = np.zeros(int(eoff[-1]), np.float32)
+            eng.explain_graphs_host(eng.make_hparams(num_epochs=EPOCHS), m0, out)
+            eng.explain_graphs_host(eng.make_hparams(num_epochs=EPOCHS, init=_abi.GX_INIT_PHILOX, seed=4), None, out)
+            print("graphvar ok", tag, float(out.sum()))
+            eng.close()
+        eng = gnnx.Engine(0)
+        eng.set_model({k: g[k] for k in util.WKEYS})
+        eng.set_graph_batch(g["adj"], g["feat"], g["label"])
+        eoff = eng.plan_graphs(gids)
+        out = np.zeros(int(eoff[-1]), np.float32)
+        eng.explain_graphs_host(eng.make_hparams(num_epochs=EPOCHS, opt=1), m0, out)
+        print("graphvar ok sgd", float(out.sum()))
+        eng.close()
+        n, d = 600, g["feat"].shape[2]
+        rng = np.random.default_rng(8)
+        adj = np.zeros((3, n, n), np.uint8); feat = np.zeros((3, n, d), np.float32)
+        for gi, k in enumerate((550, 30, 300)):
+            par = np.array([rng.integers(0, i) for i in range(1, k)])
+            adj[gi, np.arange(1, k), par] = 1; adj[gi, par, np.arange(1, k)] = 1
+            feat[gi, np.arange(k), rng.integers(0, d, k)] = 1.0
+        eng = gnnx.Engine(0)
+        eng.set_model({k: g[k] for k in util.WKEYS})
+        eng.set_graph_batch(adj, feat, np.array([0, 1, 0], np.int32))
+        eoff = eng.plan_graphs([0, 1, 2])
+        out = np.zeros(int(eoff[-1]), np.float32)
+        eng.explain_graphs_host(eng.make_hparams(num_epochs=EPOCHS, init=_abi.GX_INIT_PHILOX, seed=1), None, out)
+        print("graphvar ok large", float(out.sum()))
         eng.close()
     if "misc" in which:
         eng = util.make_engine(fx)
